@@ -16,6 +16,8 @@ streams (SURVEY 8d: L = literal-only, the headline; Z = LZ77 command streams; dy
 checked bit-exact against the raw input.  With N > 1, `scattered_e2e` times the sharded API (divans_b200.sharding.ShardedDecoder):
 rank 0 owns the whole host batch, scatters it over NVLink, every rank decodes, rank 0 gathers.
   python bench.py --workload entropy       BASELINE configs[4]: 128 x 1 MiB Bernoulli streams per GPU, p in {0.5, 0.9, 0.99}
+  python bench.py --dump-outputs DIR       also write what the last timed step decoded (rank 0) to DIR/*.npy, so that two builds
+                                           can be compared output for output (the inputs are seeded: same arguments, same inputs)
 """
 import argparse
 import json
@@ -33,6 +35,7 @@ sys.path.insert(0, ROOT)
 STREAM_BYTES = 65536
 STREAMS_PER_GPU = 4096           # N = 1 (BASELINE configs[1])
 STREAMS_PER_GPU_SCALING = 8192   # N > 1 (BASELINE configs[2]: 65536 streams at 8 GPUs)
+DUMP_STREAMS = 128               # --dump-outputs: 128 x 64 KiB decoded bytes as float32 = 32 MiB (all 4096 would be 1 GiB)
 METRIC = "decompressed MB/s (batched 64KiB streams)"
 UNIT = "MB/s"
 
@@ -247,6 +250,19 @@ def _device_decode_ms(eng, torch, dev, stream, comp, coff, clen, raw_blob, off, 
     return e0.elapsed_time(e1) / steps, eng.last_main_kernel_ms(), ok
 
 
+def dump_outputs(path, d_out, d_out_len, d_status, n):
+    """What a caller of decode_batch_device receives from one step: status and decoded length of every stream, and the decoded
+    bytes of a fixed, seeded sample of DUMP_STREAMS streams (stream_index.npy names them), one row per stream."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    pick = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_STREAMS), replace=False))
+    rows = d_out[: n * STREAM_BYTES].view(n, STREAM_BYTES)[torch.from_numpy(pick).to(d_out.device)]
+    np.save(os.path.join(path, "decoded.npy"), rows.cpu().numpy().astype(np.float32))
+    np.save(os.path.join(path, "stream_index.npy"), pick.astype(np.float64))
+    np.save(os.path.join(path, "out_len.npy"), d_out_len.cpu().numpy().astype(np.float64))
+    np.save(os.path.join(path, "status.npy"), d_status.cpu().numpy().astype(np.float64))
+
+
 def _compact(out, eoff, out_len):
     n = len(out_len)
     pad = (out_len + np.uint64(15)) & ~np.uint64(15)
@@ -338,7 +354,12 @@ def main():
     ap.add_argument("--lanes", type=int, default=int(os.environ.get("DIVANS_B200_LPS", "0")), help="lanes per stream: 16 / 8 (v2 engine), 32 / 116 (round-1 kernels); 0 = by batch size")
     ap.add_argument("--cpu-sample", type=int, default=0, help="streams in the cpu_baseline sample (0 = auto)")
     ap.add_argument("--skip-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step decoded to DIR/*.npy (float32 / float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "text"):
+        ap.error("--dump-outputs writes the outputs of the text workload on the GPU (--impl ours --workload text)")
     if args.impl == "reference":
         return run_reference_arm(args)
 
@@ -413,6 +434,8 @@ def main():
     clocks = sampler.stop()
     dev_ms = ev0.elapsed_time(ev1)
     launches = eng.launch_count - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, d_out, d_out_len, d_status, n)
     # the decode kernel's own duration (CUDA events inside the library, on the same stream), one extra untimed pass
     for _ in range(3):
         step_device()

@@ -2,12 +2,13 @@
 divANS path (SURVEY 8c).  Reference citations name the test that carries the vector."""
 import ctypes
 import hashlib
+import json
+import lzma
 import os
 
 import numpy as np
-import pytest
 
-REF = "/root/reference/testdata/"
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def test_crc32c_known_answers(oracle):
@@ -83,32 +84,15 @@ def test_dictionary_words(oracle):
 
 
 def test_transform_matches_system_brotli(oracle):
-    # cross-check our RFC 7932 transform against libbrotlicommon's BrotliTransformDictionaryWord where it is installed
-    try:
-        lib = ctypes.CDLL("libbrotlicommon.so.1")
-    except OSError:
-        pytest.skip("libbrotlicommon not present")
-    lib.BrotliGetTransforms.restype = ctypes.c_void_p
-    lib.BrotliGetDictionary.restype = ctypes.c_void_p
-    tr = lib.BrotliGetTransforms()
-    lib.BrotliTransformDictionaryWord.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_int]
-    lib.BrotliTransformDictionaryWord.restype = ctypes.c_int
-
-    class BD(ctypes.Structure):
-        _fields_ = [("sb", ctypes.c_uint8 * 32), ("off", ctypes.c_uint32 * 32), ("n", ctypes.c_size_t), ("data", ctypes.POINTER(ctypes.c_uint8))]
-    d = ctypes.cast(lib.BrotliGetDictionary(), ctypes.POINTER(BD)).contents
+    # cross-check our RFC 7932 transform against libbrotlicommon's BrotliTransformDictionaryWord: 600 random
+    # (word size, word id, transform) triples and the words it made of them (tests/golden/make_golden.py)
+    vectors = json.load(open(os.path.join(GOLD, "brotli_transforms.json")))["vectors"]
+    assert len(vectors) == 600
     L = oracle.lib()
-    rng = np.random.default_rng(7)
-    for _ in range(600):
-        ws = int(rng.integers(4, 25))
-        wid = int(rng.integers(0, 1 << d.sb[ws]))
-        t = int(rng.integers(0, 121))
-        word = ctypes.addressof(d.data.contents) + d.off[ws] + wid * ws
-        ref = np.zeros(64, np.uint8)
-        n_ref = lib.BrotliTransformDictionaryWord(ref.ctypes.data, word, ws, tr, t)
+    for ws, wid, t, ref in vectors:
         mine = np.zeros(64, np.uint8)
         n = L.dvo_dict_word(ws, wid, t, mine.ctypes.data)
-        assert n == n_ref and mine[:n].tobytes() == ref[:n].tobytes(), (ws, wid, t)
+        assert mine[:n].tobytes().hex() == ref, (ws, wid, t)
 
 
 def _cdf(oracle, vals=None):
@@ -174,27 +158,46 @@ def test_encoder_is_deterministic_against_golden(oracle, golden):
     assert rc == 0 and oracle.encode_raw(raw) == enc
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="reference tree not mounted (GPU box)")
+def _reference_ir():
+    return json.load(open(os.path.join(GOLD, "reference_ir.json")))
+
+
+def _golden_raw(oracle, golden, name):
+    # the reference's raw testdata file, as the committed fixture coded from it decodes (sha256 pinned in golden.json)
+    e = [g for g in golden if g["name"] == name][0]
+    rc, raw = oracle.decode(open(e["path"], "rb").read(), out_cap=e["raw_len"] + 64)
+    assert rc == 0 and hashlib.sha256(raw).hexdigest() == e["raw_sha256"]
+    return raw
+
+
 def test_ir_fixtures_recode_to_raw(oracle):
-    # reference src/bin/integration_test.rs:76-108
-    for name in ["alice29", "asyoulik", "random_then_unicode", "ends_with_truncated_dictionary"]:
-        raw = open(REF + name, "rb").read()
-        c = oracle.Commands.from_ir(open(REF + name + ".ir", "rb").read())
+    # reference src/bin/integration_test.rs:76-108, on the first 4000 lines of each IR file (the whole file for
+    # ends_with_truncated_dictionary): they replay to the first bytes of the reference's raw file
+    samples = _reference_ir()["samples"]
+    assert [s["name"] for s in samples] == ["alice29", "asyoulik", "random_then_unicode", "ends_with_truncated_dictionary"]
+    for s in samples:
+        text = lzma.decompress(open(os.path.join(GOLD, s["name"] + ".ir.xz"), "rb").read())
+        assert hashlib.sha256(text).hexdigest() == s["ir_sha256"], s["name"]
+        c = oracle.Commands.from_ir(text)
         rc, rec = c.recode(c.window or 22)
-        assert rc == 0 and rec == raw
+        assert rc == 0 and len(rec) == s["raw_len"] and hashlib.sha256(rec).hexdigest() == s["raw_sha256"], s["name"]
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="reference tree not mounted (GPU box)")
-def test_ratio_ceilings(oracle):
+def test_ratio_ceilings(oracle, golden):
     # reference src/bin/integration_test.rs:235-236 (alice29 <= 0.34 with brotli commands, <= 0.46 literal-only),
-    # src/bin/benchmark.rs:430-443 (random_then_unicode IR <= 0.6)
-    raw = open(REF + "alice29", "rb").read()
+    # src/bin/benchmark.rs:430-443 (random_then_unicode IR <= 0.6).  The command list of a whole IR file is the one the
+    # committed fixture coded from it carries; re-encoded, it must give the stream the reference's IR file gives.
+    raw = _golden_raw(oracle, golden, "alice29_literal_only")
     assert len(oracle.encode_raw(raw)) / len(raw) <= 0.46
-    c = oracle.Commands.from_ir(open(REF + "alice29.ir", "rb").read())
-    assert len(c.encode(oracle.options(dynamic_context_mixing=1))) / len(raw) <= 0.34
-    raw = open(REF + "random_then_unicode", "rb").read()
-    c = oracle.Commands.from_ir(open(REF + "random_then_unicode.ir", "rb").read())
-    assert len(c.encode()) / len(raw) <= 0.6
+    encodes = {e["source_ir"]: e for e in _reference_ir()["encodes"]}
+    for ir, raw_name, ceiling in [("alice29.ir", "alice29_literal_only", 0.34), ("random_then_unicode.ir", "random_then_unicode_ir", 0.6)]:
+        e = encodes["testdata/" + ir]
+        raw = _golden_raw(oracle, golden, raw_name)
+        rc, _, c = oracle.decode_cmds(open(os.path.join(GOLD, e["golden"] + ".divans"), "rb").read())
+        assert rc == 0
+        enc = c.encode(oracle.options(**e["options"]))
+        assert len(enc) == e["divans_len"] and hashlib.sha256(enc).hexdigest() == e["divans_sha256"], ir
+        assert len(enc) / len(raw) <= ceiling, ir
 
 
 def test_roundtrip_edge_cases(oracle):
@@ -257,25 +260,18 @@ def test_random_ir_roundtrip(oracle):
 # ---------------------------------------------------------------------------------------------------------------
 # The one compressed stream the reference tree holds (wasm/wasm.html:98-107): whole-bitstream pin of the oracle.
 # ---------------------------------------------------------------------------------------------------------------
-GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-
-
 def _wasm_vector():
-    import json
     vec = open(os.path.join(GOLD, "ref_wasm_example.divans"), "rb").read()
     meta = json.load(open(os.path.join(GOLD, "ref_wasm_example.json")))
     return vec, meta
 
 
 def test_reference_held_stream_fixture_is_the_reference_bytes():
-    # the committed fixture equals what wasm/wasm.html holds (checked whenever the reference tree is mounted)
-    import re
+    # the committed fixture equals what wasm/wasm.html holds: its sha256 was taken from that array when it was extracted
+    # (tests/golden/extract_wasm_vector.py)
     vec, meta = _wasm_vector()
     assert len(vec) == 113 and hashlib.sha256(vec).hexdigest() == meta["divans_sha256"]
-    html = "/root/reference/wasm/wasm.html"
-    if os.path.exists(html):
-        m = re.search(r"_example_dv_file\s*=\s*\[(.*?)\]", open(html).read(), re.S)
-        assert bytes(int(x, 16) for x in re.findall(r"0x([0-9a-fA-F]{2})", m.group(1))) == vec
+    assert meta["divans_sha256"] == "1aa983e906e5dc781f21c25baea8992c37b3fa12aa4ae45a4d847c43c476869a"
 
 
 def test_reference_held_stream_decodes_under_its_model_revision(oracle):
